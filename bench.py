@@ -24,6 +24,7 @@ cpu_baseline / --impl reference: the reference's CPU path for the same turn on t
     python bench.py --gpus 1 --steps 3 --warmup 3
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps 1 --warmup 0
+    python bench.py --gpus 1 --steps 3 --warmup 3 --dump-outputs DIR     # + what the last timed wave computed, as DIR/*.npy
 """
 from __future__ import annotations
 
@@ -41,6 +42,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True    # the benchmark leaves the tree as it found it (it may be read-only)
 
 MODEL = "small"
 AUDIO_S = 10.0
@@ -330,9 +332,13 @@ class TtsProfileWindow:
                     self.torch.cuda.cudart().cudaProfilerStop()
 
 
-def wave_device(st: Stack, pcm_dev, ev, tts_prof: "TtsProfileWindow | None" = None) -> None:
-    """One wave of S full turns as an engine-level launch sequence; stage boundaries marked with CUDA events."""
+def wave_device(st: Stack, pcm_dev, ev, tts_prof: "TtsProfileWindow | None" = None, out: "dict | None" = None) -> None:
+    """One wave of S full turns as an engine-level launch sequence; stage boundaries marked with CUDA events.  `out`, when given,
+    collects the device tensors the wave returns (token ids, codec codes, int16 audio) for wave_outputs()."""
     torch, S = st.torch, st.S
+    keep = out is not None
+    if keep:
+        out.update(stt=[], llm_first=[], llm=[], tts=[])
     dev = f"cuda:{st.dev}"
     ev["t0"].record()
     for b0 in range(0, S, 16):                                           # ---- STT
@@ -341,8 +347,10 @@ def wave_device(st: Stack, pcm_dev, ev, tts_prof: "TtsProfileWindow | None" = No
         st.whisper.encode(nb)
         wa, wb_ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         wa.record()
-        st.whisper.decode(nb, st.opts)
+        ids, _ = st.whisper.decode(nb, st.opts)
         wb_.record()
+        if keep:
+            out["stt"].append(ids)
         ev["whisper_mark"].append((wa, wb_))
     ev["stt"].record()
     firsts = []
@@ -355,27 +363,33 @@ def wave_device(st: Stack, pcm_dev, ev, tts_prof: "TtsProfileWindow | None" = No
     first = torch.cat(firsts)
     for b0 in range(0, S, st.llm_b):                                      # ---- LLM decode, llm_b sessions per launch
         sl = list(range(b0, min(S, b0 + st.llm_b)))
-        st.llm.decode(sl, first[b0:b0 + len(sl)].contiguous(), MAX_NEW - 1)
+        ids, _ = st.llm.decode(sl, first[b0:b0 + len(sl)].contiguous(), MAX_NEW - 1)
+        if keep:
+            out["llm"].append(ids)
+    if keep:
+        out["llm_first"].append(first)
     ev["llm"].record()
     eng = st.tts.engine
     text1, text2 = [3] * FIRST_SENTENCE, [5] * (MAX_NEW - FIRST_SENTENCE)
     for text, frames in ((text1, F1), (text2, F2)):                       # ---- TTS: two utterances per turn
         for s in range(S):
             eng.prefill(s, text, 2301)
+        if keep:
+            out["tts"].append([])                                         # per chunk: (codes of each launch, audio of each session)
         done, ci = 0, 0
         while done < frames:
             n = min(CHUNK, frames - done)
             if tts_prof is not None and text is text2:
                 tts_prof.chunk_begin(ci)
-            for b0 in range(0, S, st.tts_b):
-                eng.decode_frames(list(range(b0, min(S, b0 + st.tts_b))), n)
+            codes = [eng.decode_frames(list(range(b0, min(S, b0 + st.tts_b))), n) for b0 in range(0, S, st.tts_b)]
             ev["frames_mark"].append((torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)))
             a, b = ev["frames_mark"][-1]
             a.record()
-            for b0 in range(0, S, st.tts_b):
-                for wav in eng.decode_audio_batch(list(range(b0, min(S, b0 + st.tts_b))), n, LEFT_CTX):
-                    st.post.to_int16_device(wav)
+            audio = [st.post.to_int16_device(wav) for b0 in range(0, S, st.tts_b)
+                     for wav in eng.decode_audio_batch(list(range(b0, min(S, b0 + st.tts_b))), n, LEFT_CTX)]
             b.record()
+            if keep:
+                out["tts"][-1].append((codes, audio))
             if tts_prof is not None and text is text2:
                 tts_prof.chunk_end(ci)
             done += n
@@ -383,15 +397,17 @@ def wave_device(st: Stack, pcm_dev, ev, tts_prof: "TtsProfileWindow | None" = No
     ev["tts"].record()
 
 
-def run_wave(stacks, pcm_dev, evs, tts_prof=None):
+def run_wave(stacks, pcm_dev, evs, tts_prof=None, outs=None):
     """One wave on every lane at once: a host thread per lane issues the lane's launch sequence on the lane's stream; the step is
-    timed on the calling stream, from an event every lane waits for to an event that waits for every lane."""
+    timed on the calling stream, from an event every lane waits for to an event that waits for every lane.  outs: one dict per
+    lane for wave_device's `out`."""
+    outs = outs or [None] * len(stacks)
     torch = stacks[0].torch
     cur = torch.cuda.current_stream()
     start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     start.record(cur)
     if len(stacks) == 1:
-        wave_device(stacks[0], pcm_dev, evs[0], tts_prof)
+        wave_device(stacks[0], pcm_dev, evs[0], tts_prof, outs[0])
     else:
         errs, Sl = [], stacks[0].S
 
@@ -401,7 +417,7 @@ def run_wave(stacks, pcm_dev, evs, tts_prof=None):
                 torch.cuda.set_device(st.dev)
                 with st.E.lane_context(st.dev, st.lane, st.lanes):
                     torch.cuda.current_stream().wait_event(start)
-                    wave_device(st, pcm_dev[i * Sl:(i + 1) * Sl], evs[i], tts_prof)
+                    wave_device(st, pcm_dev[i * Sl:(i + 1) * Sl], evs[i], tts_prof, outs[i])
                     evs[i]["done"].record()
             except BaseException as e:  # noqa: BLE001
                 errs.append(e)
@@ -496,6 +512,28 @@ def e2e_wave(handlers, auds, S, offsets=None) -> dict:
     return {"wall_s": wall, "latency_ms": ok, "rtf": [x for x in rtf if x is not None], "errors": errs[:3]}
 
 
+DUMP_AUDIO_SAMPLES = 1 << 21      # --dump-outputs: int16 samples kept of the wave's audio (all of it is 78 MB as float32)
+
+
+def wave_outputs(outs: list) -> dict:
+    """What one wave returned (wave_device's `out` of every lane), sessions in order lane by lane, as float32 arrays: the STT and
+    LLM token ids, the codec codes of both TTS utterances, and a fixed, seeded sample of the 16 kHz int16 audio of every session
+    (the utterances one after the other) with its (session, sample) index."""
+    import torch
+    cat = torch.cat
+    res = {"stt_token_ids": cat([t for o in outs for t in o["stt"]]),
+           "llm_token_ids": cat([cat([cat(o["llm_first"])[:, None], cat(o["llm"])], 1) for o in outs])}
+    for u, name in enumerate(("first_sentence", "rest")):
+        res[f"tts_codes_{name}"] = cat([cat([cat(codes) for codes, _ in o["tts"][u]], 1) for o in outs])
+    audio = cat([torch.stack([cat([a[j] for chunks in o["tts"] for _, a in chunks]) for j in range(o["llm_first"][0].numel())])
+                 for o in outs]).cpu().numpy()
+    res = {k: v.cpu().numpy() for k, v in res.items()}
+    pick = np.sort(np.random.default_rng(0).choice(audio.size, min(audio.size, DUMP_AUDIO_SAMPLES), replace=False))
+    res["tts_audio_int16_sample"] = audio.reshape(-1)[pick]
+    res["tts_audio_int16_sample_index"] = np.stack(np.unravel_index(pick, audio.shape), 1)
+    return {k: v.astype(np.float32) for k, v in res.items()}
+
+
 LLM_STREAM_CHUNK = 4     # tokens per decode launch in the handler path: the TTS stage sees a sentence at most 4 steps late, and a
                          # first-sentence TTS request waits behind at most 4 LLM steps on the lane's stream
 
@@ -548,6 +586,9 @@ def main():
                     help="cudaProfilerStart/Stop around this many 8-frame chunks (frames + codec + post-processing) of the TTS stage only")
     ap.add_argument("--profile-region", action="store_true",
                     help="cudaProfilerStart/Stop around the device-timed region (use with ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's sessions) as DIR/<name>.npy, float32, under 64 MB; "
+                         "the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -623,7 +664,8 @@ def main():
         flush.fill_(i & 0xFF)                 # L2 flush between timed steps (not timed)
         ev = new_events()
         prof = TtsProfileWindow(torch, L, args.profile_tts_chunks) if args.profile_tts_chunks > 0 and i == 0 else None
-        spans.append(run_wave(stacks, pcm_dev, ev, prof))
+        outs = [{} for _ in stacks] if args.dump_outputs and rank == 0 and i == args.steps - 1 else None
+        spans.append(run_wave(stacks, pcm_dev, ev, prof, outs))
         evs.append(ev[0])                     # stage boundaries: lane 0's (the lanes run the same sequence side by side)
     barrier()
     if args.profile_region:
@@ -631,6 +673,14 @@ def main():
     wall_s = time.perf_counter() - t_wall
     launches = E.launch_count(local_rank, reset=True)
     log(f"timed region done: {wall_s:.2f} s for {args.steps} wave(s), {launches} launches")
+    if args.dump_outputs and rank == 0:
+        dumped = wave_outputs(outs)
+        assert sum(a.nbytes for a in dumped.values()) <= 64 << 20
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
+        log(f"outputs of the last timed wave written to {args.dump_outputs}: " + ", ".join(f"{k} {list(a.shape)}" for k, a in dumped.items()))
+        del dumped, outs
 
     def stage(ev, a, b):
         return ev[a].elapsed_time(ev[b])

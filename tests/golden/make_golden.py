@@ -2,6 +2,7 @@
 
 Run in the builder container (transformers 5.5.0, CPU):
     python tests/golden/make_golden.py [whisper|llama|code2wav|qwen3tts|all]
+    PYTHONPATH=<speech-to-speech checkout>/src python tests/golden/make_golden.py tts_handler
 
 The reference holds no golden mel/logits/ids for this path (SURVEY.md section 4), so the
 pin is the upstream model code itself: WhisperFeatureExtractor + WhisperForConditionalGeneration
@@ -13,6 +14,7 @@ from __future__ import annotations
 
 import os
 import sys
+import zlib
 
 import numpy as np
 
@@ -255,6 +257,14 @@ def code2wav_golden(name: str = "micro"):
     print("wrote", path, wav.shape, float(np.abs(wav).max()))
 
 
+def sample_logits(logits: np.ndarray, keep: float = 0.5, top: int = 8, seed: int = 5) -> np.ndarray:
+    """Keep the file under 1 MB: every row keeps its `top` largest logits (the top-1 / top-2 margins stay exact) and a seeded
+    `keep` share of the other entries; the rest become NaN."""
+    kept = np.random.default_rng(seed).random(logits.shape) < keep
+    np.put_along_axis(kept, np.argsort(logits, axis=-1)[..., -top:], True, axis=-1)
+    return np.where(kept, logits, np.float32(np.nan)).astype(np.float32)
+
+
 def qwen3tts_golden(name: str = "micro", text_len: int = 6, max_frames: int = 10):
     """Talker + code predictor of the published cousin (`Qwen3OmniMoeTalkerForConditionalGeneration`, transformers) at
     seeded weights, driven exactly like `Qwen3OmniMoeForConditionalGeneration.generate` step 2 drives it, with the two
@@ -335,14 +345,53 @@ def qwen3tts_golden(name: str = "micro", text_len: int = 6, max_frames: int = 10
     path = os.path.join(OUT, f"qwen3tts_{name}.npz")
     np.savez_compressed(path, text_ids=np.asarray(text_ids, np.int32), speaker=speaker, codes=codes.astype(np.int32),
                         code0_all=res.sequences[0].numpy().astype(np.int32), talker_logits=t_scores.astype(np.float32),
-                        predictor_logits=np.stack(pred_scores).astype(np.float32), prompt_embeds=embeds[0].numpy().astype(np.float32),
+                        predictor_logits=sample_logits(np.stack(pred_scores).astype(np.float32)),
+                        prompt_embeds=embeds[0].numpy().astype(np.float32),
                         trailing=trailing[0].numpy().astype(np.float32), max_frames=max_frames,
                         transformers_version=__import__("transformers").__version__)
     print("wrote", path, codes.shape, codes[:2].tolist(), "code0", res.sequences[0].tolist())
 
 
+TTS_HANDLER_SIZES = (1, 480, 1920, 15360, 48001)
+BUDGET_ALPHABET = list("abcdefghij klmnop, qrst. uvw! xyz? 上海是一座城市，。") + [" "] * 6
+BUDGET_CASES = ((8, 1536), (4, 700), (1, 5000))
+
+
+def tts_handler_golden():
+    """What the upstream Qwen3TTSHandler (huggingface/speech-to-speech, TTS/qwen3_tts_handler.py) returns from
+    `_resample_to_pipeline_sr` / `_to_int16` on seeded audio and from `_estimate_max_new_tokens` on seeded random text.
+    Needs the upstream sources importable, e.g. PYTHONPATH=<speech-to-speech checkout>/src (not part of `all`)."""
+    from speech_to_speech.TTS.qwen3_tts_handler import Qwen3TTSHandler
+
+    h = object.__new__(Qwen3TTSHandler)
+    out = {}
+    rng = np.random.default_rng(7)       # the inputs are regenerated from these seeds by tests/test_oracle_tts.py
+    for n in TTS_HANDLER_SIZES:
+        x = (0.4 * rng.standard_normal(n)).astype(np.float32)
+        y = h._resample_to_pipeline_sr(x, 24000)
+        out[f"resampled_{n}"], out[f"int16_{n}"] = y, h._to_int16(y)
+    x = (0.2 * np.random.default_rng(0).standard_normal(4410)).astype(np.float32)
+    y = h._resample_to_pipeline_sr(x, 44100)
+    out["resampled_44100"], out["int16_44100"] = y, h._to_int16(y)
+    rng = np.random.default_rng(0)       # the texts too (tests/test_tts_handler.py); their CRC-32s are stored to check that
+    crcs, budgets = [], []
+    for chunk, cap in BUDGET_CASES:
+        h.streaming_chunk_size, h.max_new_tokens = chunk, cap
+        for _ in range(200):
+            text = "".join(rng.choice(BUDGET_ALPHABET, int(rng.integers(0, 900))))
+            crcs.append(zlib.crc32(text.encode()))
+            budgets.append(h._estimate_max_new_tokens(text))
+    path = os.path.join(OUT, "tts_handler_reference.npz")
+    np.savez_compressed(path, budget_cases=np.asarray(BUDGET_CASES, np.int32),
+                        budget_text_crc32=np.asarray(crcs, np.uint32).reshape(len(BUDGET_CASES), -1),
+                        budgets=np.asarray(budgets, np.int32).reshape(len(BUDGET_CASES), -1), **out)
+    print("wrote", path, os.path.getsize(path), "bytes")
+
+
 if __name__ == "__main__":
     what = sys.argv[1] if len(sys.argv) > 1 else "all"
+    if what == "tts_handler":
+        tts_handler_golden()
     if what in ("whisper", "all"):
         for n in WHISPER_CASES:
             whisper_golden(n)

@@ -1,5 +1,5 @@
 """Host-side pieces of bench.py that run without a GPU: the workload description both arms print, the byte models behind the
-roofline numbers, the ncu window over TTS chunks, and the lane fan-out of a wave."""
+roofline numbers, the ncu window over TTS chunks, the lane fan-out of a wave, and the arrays --dump-outputs writes."""
 import importlib.util
 import os
 import subprocess
@@ -23,7 +23,7 @@ def bench():
 def test_cli_parses_and_documents_the_contract_flags():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--sessions", "--lanes"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--sessions", "--lanes", "--dump-outputs"):
         assert flag in out.stdout
 
 
@@ -112,3 +112,31 @@ def test_e2e_wave_runs_the_stages_in_their_own_threads_and_honours_offsets(bench
     for i in (0, 1):
         assert hs[i][2].spoken == [(bench.FIRST_SENTENCE, bench.F1), (bench.MAX_NEW - bench.FIRST_SENTENCE, bench.F2)]
     assert all(x > 0 for x in r["rtf"])
+
+
+def test_wave_outputs_put_every_session_in_order_as_float32(bench, monkeypatch):
+    """bench.wave_outputs on what wave_device collects for 2 lanes x 3 sessions (two LLM / TTS launches per lane, two TTS
+    utterances of 2 and 1 chunks): every value names its session, so the order across lanes, launches and chunks is checked."""
+    import numpy as np
+    import torch
+    monkeypatch.setattr(bench, "DUMP_AUDIO_SAMPLES", 50)
+
+    def lane(l):
+        sid = torch.arange(3, dtype=torch.int32) + 3 * l
+        ids = lambda rows, n: sid[rows, None].repeat(1, n)
+        chunk = lambda n: ([ids(slice(0, 2), n * 16).view(2, n, 16), ids(slice(2, 3), n * 16).view(1, n, 16)],
+                           [torch.full((4 * n,), int(s), dtype=torch.int16) for s in sid])
+        return {"stt": [ids(slice(0, 3), 128)], "llm_first": [sid], "llm": [ids(slice(0, 2), 127), ids(slice(2, 3), 127)],
+                "tts": [[chunk(8), chunk(2)], [chunk(5)]]}
+    out = bench.wave_outputs([lane(0), lane(1)])
+    assert all(a.dtype == np.float32 for a in out.values())
+    col = np.arange(6, dtype=np.float32)[:, None]
+    assert np.array_equal(out["stt_token_ids"], np.repeat(col, 128, 1))
+    assert np.array_equal(out["llm_token_ids"], np.repeat(col, 128, 1))
+    assert out["tts_codes_first_sentence"].shape == (6, 10, 16) and out["tts_codes_rest"].shape == (6, 5, 16)
+    assert (out["tts_codes_first_sentence"] == col[:, :, None]).all() and (out["tts_codes_rest"] == col[:, :, None]).all()
+    idx = out["tts_audio_int16_sample_index"]
+    assert idx.shape == (50, 2) and idx[:, 1].max() < 4 * 15 and len({tuple(r) for r in idx.tolist()}) == 50
+    assert np.array_equal(out["tts_audio_int16_sample"], idx[:, 0])
+    again = bench.wave_outputs([lane(0), lane(1)])
+    assert np.array_equal(again["tts_audio_int16_sample_index"], idx)          # a fixed sample: runs compare element for element

@@ -1,9 +1,7 @@
-"""CPU: the drop-in boundary.  With the reference on the path (builder container) our handlers must subclass ITS
-base classes, register in ITS backend registry and honour ITS process() contract; the device work is replaced
-by a fake engine exactly the way the reference's own tests fake their models
+"""CPU: the drop-in boundary.  With the reference (the upstream `speech_to_speech` package, oracle/upstream.py) importable our handlers must
+subclass ITS base classes, register in ITS backend registry and honour ITS process() contract; the device work is
+replaced by a fake engine exactly the way the reference's own tests fake their models
 (T/test_whisper_language_detection.py:52-141).  Without the reference the same contract is checked on the mirror."""
-import os
-import sys
 from queue import Queue
 from threading import Event, Thread
 from types import SimpleNamespace
@@ -11,10 +9,9 @@ from types import SimpleNamespace
 import numpy as np
 import pytest
 
-REF_SRC = "/root/reference/src"
-HAVE_REF = os.path.isdir(REF_SRC)
-if HAVE_REF and REF_SRC not in sys.path:
-    sys.path.insert(0, REF_SRC)
+from oracle import upstream
+
+HAVE_REF = upstream.importable()
 
 from speech_to_speech_b200.host import resolve  # noqa: E402
 from speech_to_speech_b200.handlers import whisper_stt_handler as WH  # noqa: E402
@@ -214,7 +211,7 @@ def test_token_table_from_generation_config():
     assert t.lang_to_id == {"en": 50259, "de": 50261, "yue": 50358} and t.suppress == [1, 2] and t.eos == 50257
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present")
+@pytest.mark.skipif(not HAVE_REF, reason="the upstream speech_to_speech package is not available")
 def test_registers_in_the_reference_backend_registry():
     import speech_to_speech_b200.registry as r
     specs = r.register()
@@ -225,7 +222,7 @@ def test_registers_in_the_reference_backend_registry():
     assert cfg["model_name"] == "random:small" and cfg["device"] == "cuda" and cfg["gen_kwargs"]["max_new_tokens"] == 128
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present")
+@pytest.mark.skipif(not HAVE_REF, reason="the upstream speech_to_speech package is not available")
 def test_tts_spec_and_overrides_cover_all_three_slots():
     """`b200-qwen3` reuses the reference's Qwen3TTSHandlerArguments / prefix; install_overrides() swaps the classes behind the
     unchanged names whisper / transformers / qwen3 (the lazy factories resolve to our modules, nothing is imported yet)."""
@@ -252,7 +249,7 @@ def test_tts_spec_and_overrides_cover_all_three_slots():
             d.clear(); d.update(s)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present")
+@pytest.mark.skipif(not HAVE_REF, reason="the upstream speech_to_speech package is not available")
 def test_llm_handler_implements_the_reference_hooks():
     from speech_to_speech_b200.handlers import language_model_handler as LH
     from speech_to_speech.LLM.language_model import BaseLanguageModelHandler

@@ -3,19 +3,16 @@
 fake that replays a scripted token sequence (the reference's tests fake the model the same way, T/test_voice_prompt.py).
 Asserts the order LLMResponseChunk ... TokenUsage, EndOfResponse, the reference's prompt-token count, enable_thinking=False,
 cancellation through cancel_scope and through a prefetch transaction's abort."""
-import os
-import sys
 from queue import Queue
 from threading import Event
 from types import SimpleNamespace
 
 import pytest
 
-REF_SRC = "/root/reference/src"
-HAVE_REF = os.path.isdir(REF_SRC)
-pytestmark = pytest.mark.skipif(not HAVE_REF, reason="reference tree not present (GPU box)")
-if HAVE_REF and REF_SRC not in sys.path:
-    sys.path.insert(0, REF_SRC)
+from oracle import upstream
+
+# the request lifecycle (Chat, messages, cancel scopes) is the reference's own code: those tests need it importable
+needs_reference = pytest.mark.skipif(not upstream.importable(), reason="the upstream speech_to_speech package is not available")
 
 
 class FakeTokenizer:
@@ -117,6 +114,7 @@ def _request(text="tell me something", **kw):
     return GenerateResponseRequest(runtime_config=RuntimeConfig(chat=chat), **kw), chat
 
 
+@needs_reference
 def test_request_flows_through_process_in_the_reference_order(monkeypatch):
     from speech_to_speech.pipeline.messages import EndOfResponse, LLMResponseChunk, TokenUsage
     h, tok, eng = _handler(monkeypatch, "Hello there. How are you today?")
@@ -141,6 +139,7 @@ def test_request_flows_through_process_in_the_reference_order(monkeypatch):
     assert eng.decode_calls >= 3       # the reply was produced in chunks of 2 tokens
 
 
+@needs_reference
 def test_cancel_scope_stops_generation_between_chunks(monkeypatch):
     from speech_to_speech.pipeline.cancel_scope import CancelScope
     from speech_to_speech.pipeline.messages import EndOfResponse, LLMResponseChunk
@@ -158,6 +157,7 @@ def test_cancel_scope_stops_generation_between_chunks(monkeypatch):
     assert 1 <= n_chunks < 8 and eng.decode_calls < 8
 
 
+@needs_reference
 def test_prefetch_abort_is_registered_and_stops_the_stream(monkeypatch):
     h, tok, eng = _handler(monkeypatch, "A b c d e f g h i j k l m n o p.")
     from speech_to_speech.LLM.language_model import StreamContext

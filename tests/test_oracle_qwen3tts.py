@@ -41,7 +41,10 @@ def test_codes_bit_exact_and_logits_close(gold, model):
     fin = np.isfinite(gold["talker_logits"])
     assert np.array_equal(fin, np.isfinite(t_logits))           # the same ids are suppressed
     assert np.abs(t_logits[fin] - gold["talker_logits"][fin]).max() < 2e-4
-    assert np.abs(p_logits[: F - 1] - gold["predictor_logits"]).max() < 2e-4
+    # the golden keeps each row's top logits and a seeded half of the rest (NaN elsewhere, make_golden.sample_logits)
+    kept = ~np.isnan(gold["predictor_logits"])
+    assert kept.mean() > 0.5 and np.isfinite(p_logits[: F - 1]).all()
+    assert np.abs(p_logits[: F - 1][kept] - gold["predictor_logits"][kept]).max() < 2e-4
 
 
 def test_suppress_list_is_the_cousins(model):

@@ -1,15 +1,13 @@
-"""CPU: the TTS post-processing oracle (oracle/tts_post_ref.py) against scipy and -- when the reference tree is present --
-against the reference handler's own helper methods (`Qwen3TTSHandler._resample_to_pipeline_sr`, `_to_int16`,
-TTS/qwen3_tts_handler.py:612-613, 674-680).  Bit-exact: the CUDA kernel is then held to the same vectors on the GPU."""
+"""CPU: the TTS post-processing oracle (oracle/tts_post_ref.py) against scipy and against what the reference handler's own
+helper methods (`Qwen3TTSHandler._resample_to_pipeline_sr`, `_to_int16`, TTS/qwen3_tts_handler.py:612-613, 674-680)
+returned, stored in tests/golden/tts_handler_reference.npz.  Bit-exact: the CUDA kernel is then held to the same vectors
+on the GPU."""
 import os
-import sys
 
 import numpy as np
 import pytest
 
 from oracle import tts_post_ref as T
-
-REF_SRC = "/root/reference/src"
 
 
 @pytest.mark.parametrize("n", [1, 2, 3, 7, 61, 100, 333, 1919, 1920])
@@ -36,43 +34,43 @@ def test_stream_blocks_trims_leading_silence_and_pads_the_tail():
     assert len(flat) == 13 * 512 and np.abs(flat[:6400]).max() > 3000 and not flat[6400:].any()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="reference tree not present (GPU box)")
-def test_oracle_equals_the_reference_handler_helpers():
-    sys.path.insert(0, REF_SRC)
-    try:
-        from speech_to_speech.TTS.qwen3_tts_handler import Qwen3TTSHandler
-    except Exception as e:  # optional heavy deps of the handler module missing
-        pytest.skip(f"reference TTS handler not importable here: {e}")
-    finally:
-        sys.path.remove(REF_SRC)
-    h = object.__new__(Qwen3TTSHandler)
+@pytest.fixture(scope="module")
+def upstream(golden_dir):
+    """What the upstream handler's own helpers returned (tests/golden/make_golden.py tts_handler)."""
+    return np.load(os.path.join(golden_dir, "tts_handler_reference.npz"))
+
+
+def _handler_base():
+    """The class the TTS handler slot builds on: the upstream Qwen3TTSHandler when installed, the mirror otherwise."""
+    from speech_to_speech_b200.handlers.qwen3_tts_handler import _base_class
+    return _base_class()
+
+
+def test_oracle_equals_the_reference_handler_helpers(upstream):
+    base = _handler_base()
+    h = object.__new__(base)
     rng = np.random.default_rng(7)
     for n in (1, 480, 1920, 15360, 48001):
         x = (0.4 * rng.standard_normal(n)).astype(np.float32)
-        ref16k = Qwen3TTSHandler._resample_to_pipeline_sr(h, x, 24000)
+        ref16k, ref_int16 = upstream[f"resampled_{n}"], upstream[f"int16_{n}"]
         assert np.array_equal(T.resample_to_16k(x, 24000), ref16k)
-        assert np.array_equal(T.to_int16(ref16k), Qwen3TTSHandler._to_int16(h, ref16k))
-        assert np.array_equal(T.postproc(x), Qwen3TTSHandler._to_int16(h, ref16k))
+        assert np.array_equal(T.to_int16(ref16k), ref_int16)
+        assert np.array_equal(T.postproc(x), ref_int16)
+        assert np.array_equal(base._resample_to_pipeline_sr(h, x, 24000), ref16k)
+        assert np.array_equal(base._to_int16(h, ref16k), ref_int16)
     same = rng.standard_normal(100).astype(np.float32)
-    assert Qwen3TTSHandler._resample_to_pipeline_sr(h, same, 16000) is same  # pipeline rate passes through untouched
+    assert base._resample_to_pipeline_sr(h, same, 16000) is same  # pipeline rate passes through untouched
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="reference tree not present (GPU box)")
-def test_patched_tts_handler_keeps_the_reference_pinned_token_budgets():
+def test_patched_tts_handler_keeps_the_reference_pinned_token_budgets(upstream):
     """The only golden values the reference's tests hold on this path are `_estimate_max_new_tokens` = 360 / 576 / cap
     (tests/test_qwen3_tts_handler_backend.py:915-964).  The handler class with the GPU post-processing patched in must
-    still produce them (the estimator stays the reference's own Python) and must leave non-24 kHz audio on the scipy path."""
-    sys.path.insert(0, REF_SRC)
-    try:
-        from speech_to_speech.TTS.qwen3_tts_handler import Qwen3TTSHandler
-    except Exception as e:
-        pytest.skip(f"reference TTS handler not importable here: {e}")
-    finally:
-        sys.path.remove(REF_SRC)
+    still produce them (the estimator stays the base class's own Python) and must leave non-24 kHz audio on the scipy path."""
     from speech_to_speech_b200.handlers.qwen3_tts_postproc import patch_handler_class
 
-    cls = patch_handler_class(Qwen3TTSHandler)
-    assert issubclass(cls, Qwen3TTSHandler)
+    base = _handler_base()
+    cls = patch_handler_class(base)
+    assert issubclass(cls, base)
     h = object.__new__(cls)
     h.streaming_chunk_size, h.max_new_tokens = 8, 1536
     long_text = " ".join(["This is a deliberately long sentence for the Qwen3 TTS budget estimator."] * 12)
@@ -89,6 +87,5 @@ def test_patched_tts_handler_keeps_the_reference_pinned_token_budgets():
     assert h._estimate_max_new_tokens(long_text) == 400
     # audio that is not 24 kHz never touches the GPU path: identical to the reference's scipy result
     x = (0.2 * np.random.default_rng(0).standard_normal(4410)).astype(np.float32)
-    ref = Qwen3TTSHandler._resample_to_pipeline_sr(object.__new__(Qwen3TTSHandler), x, 44100)
-    assert np.array_equal(h._resample_to_pipeline_sr(x, 44100), ref)
-    assert np.array_equal(h._to_int16(ref), Qwen3TTSHandler._to_int16(object.__new__(Qwen3TTSHandler), ref))
+    assert np.array_equal(h._resample_to_pipeline_sr(x, 44100), upstream["resampled_44100"])
+    assert np.array_equal(h._to_int16(upstream["resampled_44100"]), upstream["int16_44100"])

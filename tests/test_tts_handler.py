@@ -1,16 +1,19 @@
 """CPU contract tests of the B200 TTS handler slot with a fake model object (the reference's own test strategy: bypass the
 device, inject fakes -- T/test_qwen3_tts_handler_backend.py:18-19, 756-762).  Both base classes are exercised: the reference's
-Qwen3TTSHandler when importable, and the mirror used on machines without /root/reference."""
+Qwen3TTSHandler when the upstream `speech_to_speech` package is importable (oracle/upstream.py), and the mirror used without it."""
 import importlib
 import os
 import sys
+import zlib
 from queue import Queue
 from threading import Event
 
 import numpy as np
 import pytest
 
-REF_SRC = "/root/reference/src"
+from oracle import upstream
+
+HAVE_UPSTREAM = upstream.importable()
 LONG = " ".join(["This is a deliberately long sentence for the Qwen3 TTS budget estimator."] * 12)
 CJK_SHORT = "我懂，心情不好时会让人特别疲惫。"
 CJK_LONG = ("上海是一座充满活力的现代化大都市，既有繁华的金融中心和摩天大楼，也有老城厢的弄堂风情"
@@ -46,28 +49,21 @@ def _handler_module(use_reference: bool):
     """Import handlers.qwen3_tts_handler against the reference base or the mirror base."""
     for m in [k for k in sys.modules if k.startswith("speech_to_speech_b200.handlers.qwen3_tts_handler")]:
         del sys.modules[m]
-    had = REF_SRC in sys.path
-    if use_reference:
-        if not os.path.isdir(REF_SRC):
-            pytest.skip("reference tree not present")
-        if not had:
-            sys.path.insert(0, REF_SRC)
-    else:
-        if had:
-            sys.path.remove(REF_SRC)
-    # the mirror base is only chosen when `speech_to_speech` cannot be imported: hide the already-imported modules for the
-    # duration of the import and PUT THEM BACK, so that other test modules keep seeing the class objects they imported
+    if use_reference and not HAVE_UPSTREAM:
+        pytest.skip("the upstream speech_to_speech package is not available")
+    # the mirror base is only chosen when `speech_to_speech` cannot be imported: block it (a None entry in sys.modules) for
+    # the duration of the import and PUT the already-imported modules BACK, so that other test modules keep seeing the class
+    # objects they imported
     hidden = {}
     if not use_reference:
         for m in [k for k in sys.modules if k == "speech_to_speech" or k.startswith("speech_to_speech.")]:
             hidden[m] = sys.modules.pop(m)
+        sys.modules["speech_to_speech"] = None
     try:
         mod = importlib.import_module("speech_to_speech_b200.handlers.qwen3_tts_handler")
     finally:
-        if use_reference and not had:
-            sys.path.remove(REF_SRC)
-        if not use_reference and had:
-            sys.path.insert(0, REF_SRC)
+        if not use_reference:
+            del sys.modules["speech_to_speech"]
         for m in [k for k in sys.modules if (k == "speech_to_speech" or k.startswith("speech_to_speech.")) and k in hidden]:
             del sys.modules[m]
         sys.modules.update(hidden)
@@ -153,26 +149,20 @@ def test_token_budget_goldens_of_the_reference(monkeypatch, use_reference):
     assert h._estimate_max_new_tokens("") == 360
 
 
-def test_mirror_budget_equals_the_reference_function_on_random_text():
-    if not os.path.isdir(REF_SRC):
-        pytest.skip("reference tree not present")
-    sys.path.insert(0, REF_SRC)
-    try:
-        from speech_to_speech.TTS.qwen3_tts_handler import Qwen3TTSHandler
-    except Exception as e:
-        pytest.skip(f"reference handler not importable: {e}")
-    finally:
-        sys.path.remove(REF_SRC)
+def test_mirror_budget_equals_the_reference_function_on_random_text(golden_dir):
+    """The mirror's `_estimate_max_new_tokens` against the budgets the reference's Qwen3TTSHandler gave for the same seeded
+    random texts (tests/golden/make_golden.py tts_handler)."""
     from speech_to_speech_b200.host.mirror_tts import MirrorQwen3TTSHandler
-    a, b = object.__new__(Qwen3TTSHandler), object.__new__(MirrorQwen3TTSHandler)
+    gold = np.load(os.path.join(golden_dir, "tts_handler_reference.npz"))
+    b = object.__new__(MirrorQwen3TTSHandler)
     rng = np.random.default_rng(0)
     alphabet = list("abcdefghij klmnop, qrst. uvw! xyz? 上海是一座城市，。") + [" "] * 6
-    for chunk, cap in ((8, 1536), (4, 700), (1, 5000)):
-        a.streaming_chunk_size = b.streaming_chunk_size = chunk
-        a.max_new_tokens = b.max_new_tokens = cap
-        for _ in range(200):
+    for (chunk, cap), crcs, budgets in zip(gold["budget_cases"].tolist(), gold["budget_text_crc32"], gold["budgets"]):
+        b.streaming_chunk_size, b.max_new_tokens = chunk, cap
+        for crc, budget in zip(crcs.tolist(), budgets.tolist()):
             text = "".join(rng.choice(alphabet, int(rng.integers(0, 900))))
-            assert a._estimate_max_new_tokens(text) == b._estimate_max_new_tokens(text), text
+            assert zlib.crc32(text.encode()) == crc            # the same text the reference was given
+            assert b._estimate_max_new_tokens(text) == budget, text
 
 
 @pytest.mark.parametrize("use_reference", [True, False])
